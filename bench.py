@@ -7,10 +7,13 @@ statistics kernel -- the kernel the 70 %-of-HBM-roofline target is quoted on) an
 quantizer sites (per-channel symmetric 8-bit).  A "step" is one pass over all 109 sites on
 synthetic tensors of exactly those shapes.  metric = fake-quant forward Gelem/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); the path has no exchange step, so ranks are
 independent replicas (weak scaling) and only the timing barrier uses NCCL.
+
+--dump-outputs DIR writes what rank 0's last timed step computed as DIR/<name>.npy (float32), so that
+two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 import argparse
 import ctypes
@@ -73,6 +76,33 @@ def numel(shape):
     for d in shape:
         n *= d
     return n
+
+
+DUMP_SAMPLE = 1 << 16  # values written per site: 109 sites stay below 30 MB (a step's outputs are 11 GB)
+
+
+def dump_outputs(out_dir, acts, weights, mm_states):
+    """Write what a step hands its caller: every site's QDQ output (act_qdq_NN / weight_qdq_NN, in site order;
+    the whole tensor when it has at most DUMP_SAMPLE elements, else the values at DUMP_SAMPLE positions drawn from
+    a fixed seed, sorted) and the (min, max) of the 55 fused MinMax observers (act_minmax, [55, 2])."""
+    import numpy as np
+
+    from sparsebit_b200 import ops
+
+    os.makedirs(out_dir, exist_ok=True)
+    g = torch.Generator().manual_seed(0)
+
+    def sample(t):
+        flat = t.reshape(-1)
+        if flat.numel() <= DUMP_SAMPLE:
+            return flat
+        return flat[torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=g).sort().values.to(flat.device)]
+
+    for prefix, sites in (("act_qdq", acts), ("weight_qdq", weights)):
+        for i, site in enumerate(sites):
+            np.save(os.path.join(out_dir, f"{prefix}_{i:02d}.npy"), sample(site[1]).cpu().numpy())
+    mn, mx = ops.minmax_read(mm_states)
+    np.save(os.path.join(out_dir, "act_minmax.npy"), torch.stack([mn, mx], dim=1).cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -617,7 +647,12 @@ def main():
     ap.add_argument("--no-gptq", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[0] / [2] / [3] blocks and the observer / sparser CPU baselines")
     ap.add_argument("--no-graphs", action="store_true", help="enqueue the 109 launches eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference_arm(args)
@@ -756,6 +791,8 @@ def main():
     total_ms = float(tmax)
     ms_per_step = total_ms / args.steps
     value = world * step_elems / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, acts, weights, mm_states)
 
     # parity spot check of what was just timed (fused kernel's min/max state, on-grid outputs)
     mn, mx = (torch.empty(1, device=dev), torch.empty(1, device=dev))
