@@ -73,6 +73,17 @@ def ste_backward(x, scale, zero_point, grad_y, qmin, qmax, ch_axis=0, rounding=0
     (fake_quant_tensor.cu:264), i.e. vq == qmax counts as clipped for the zero-point gradient only (SURVEY Q4).
     Pinned to MySTE.backward outputs (tests/golden/bwd.npz) and, on the GPU box, to the reference's own
     kernels (tests/test_gpu_reference_ext.py).  Returns gx (fp32), gs, gzp (fp64, shape [C] or [1])."""
+    gx, gs_e, gz_e = ste_backward_terms(x, scale, zero_point, grad_y, qmin, qmax, ch_axis, rounding, gzp_open_top)
+    nch = np.asarray(scale).size
+    if nch == 1:
+        return gx, np.array([gs_e.sum()]), np.array([gz_e.sum()])
+    axes = tuple(a for a in range(gx.ndim) if a != ch_axis)
+    return gx, gs_e.sum(axis=axes), gz_e.sum(axis=axes)
+
+
+def ste_backward_terms(x, scale, zero_point, grad_y, qmin, qmax, ch_axis=0, rounding=0, gzp_open_top=False):
+    """``ste_backward`` before the reductions: gx (fp32) and the per-element fp64 terms of gs and gzp, shaped like x
+    (a tolerance for the sums can be stated against the L1 norm of their terms)."""
     x = np.asarray(x, dtype=F32)
     gy = np.asarray(grad_y, dtype=F32)
     s = _bcast(scale, x, ch_axis)
@@ -88,11 +99,7 @@ def ste_backward(x, scale, zero_point, grad_y, qmin, qmax, ch_axis=0, rounding=0
     gs_e = term.astype(np.float64) * gy.astype(np.float64)
     inside_z = inside & (vq < F32(qmax)) if gzp_open_top else inside
     gz_e = np.where(inside_z, 0.0, (-s).astype(np.float64) * gy.astype(np.float64))
-    nch = np.asarray(scale).size
-    if nch == 1:
-        return gx, np.array([gs_e.sum()]), np.array([gz_e.sum()])
-    axes = tuple(a for a in range(x.ndim) if a != ch_axis)
-    return gx, gs_e.sum(axis=axes), gz_e.sum(axis=axes)
+    return gx, gs_e, gz_e
 
 
 # --------------------------------------------------------------------------------------------

@@ -474,7 +474,9 @@ __global__ void __launch_bounds__(kThreads) select_scan_kernel(unsigned long lon
     if (threadIdx.x == 0) {
       unsigned long long b = s_found[0];
       unsigned long long below = s_found[1];
-      if (b == 0xFFFFFFFFFFFFFFFFull) {  // rank beyond the population: clamp to the last non-empty bin
+      if (b == 0xFFFFFFFFFFFFFFFFull) {  // rank beyond the population: no bin holds it, bin 0 is taken and the value
+        // read back is meaningless.  Callers keep ranks below the row length (ops.kth_value rejects k >= n,
+        // percentile_ranks_kernel clamps to the row total).
         b = 0;
         below = 0;
       }

@@ -99,16 +99,19 @@ BWD_GZP_CLOSED = 1  # include/sparsebit_b200.h SB200_BWD_GZP_CLOSED
 
 
 def qdq_backward(x, scale, zero_point, grad_y, qmin, qmax, ch_axis=None, rounding=0, need_gs=True, need_gzp=True,
-                 gzp_closed=False):
+                 gzp_closed=False, out=None):
     """Returns (gx, gs, gzp); gs / gzp shaped like scale / zero_point (zeros when not requested,
     like the reference which returns zeros_like, fake_quant_tensor.cu:147-149).  Per-channel zero-point
     gradient: by default the reference kernel's rule (vq == qmax counts as clipped, fake_quant_tensor.cu:264);
-    ``gzp_closed=True`` selects MySTE.backward's closed interval (quant_tensor.py:62-69)."""
+    ``gzp_closed=True`` selects MySTE.backward's closed interval (quant_tensor.py:62-69).  ``out``: optional
+    contiguous fp32 tensor shaped like x that receives gx."""
     lib = _lib.load()
     _req(x, "data"), _req(scale, "scale"), _req(zero_point, "zero_point"), _req(grad_y, "grad")
     if grad_y.shape != x.shape:
         raise SparsebitB200Error("grad_y must have the shape of data")
-    gx = torch.empty_like(x)
+    gx = torch.empty_like(x) if out is None else _req(out, "grad_x")
+    if gx.shape != x.shape:
+        raise SparsebitB200Error("out must have the shape of data")
     gs = torch.zeros_like(scale)
     gzp = torch.zeros_like(zero_point)
     if ch_axis is None:
@@ -449,6 +452,8 @@ class RadixSelect:
 
 def kth_value(x, k, key_mode=0):
     """k-th smallest (0-based) of a flat tensor, exact; key_mode 1 ranks |x|."""
+    if not 0 <= int(k) < x.numel():
+        raise SparsebitB200Error(f"kth_value: k must be in [0, {x.numel()}) (got {k})")
     rs = RadixSelect(1, 1, x.device, key_mode)
     rs.set_ranks(torch.tensor([k], dtype=torch.int64, device=x.device))
     x2 = x.reshape(1, -1)
