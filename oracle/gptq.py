@@ -118,13 +118,20 @@ def pack_bits(w, scale, zero, bit):
     g = scale.shape[1]
     zeros = (zero * scale).astype(F32)
     iw = np.rint(((w.reshape(n, g, -1) + zeros[:, :, None]) / scale[:, :, None]).astype(F32)).astype(np.int64)
-    iw = iw.reshape(n, k).T.astype(np.uint64)  # [K, N]
+    return pack_values(iw.reshape(n, k).T, bit), scale.astype(F32), zeros
+
+
+def pack_values(iw, bit):
+    """The packing step of QuantLinear.pack alone: unsigned integer weights iw [K, N] (< 2^bit) ->
+    int32 qweight [packed_rows(K, bit), N].  Any K: no group structure is involved."""
+    iw = np.asarray(iw).astype(np.uint64)
+    k, n = iw.shape
     q = np.zeros((packed_rows(k, bit), n), dtype=np.uint64)
     for i, (row, shift, srow, sshift) in enumerate(_bit_slots(bit, k)):
         q[row] |= (iw[i] << np.uint64(shift)) & np.uint64(0xFFFFFFFF)
         if srow is not None:
             q[srow] |= iw[i] >> np.uint64(sshift)
-    return q.astype(np.uint32).view(np.int32), scale.astype(F32), zeros
+    return q.astype(np.uint32).view(np.int32)
 
 
 def unpack_bits(qweight, k, bit):

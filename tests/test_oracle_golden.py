@@ -89,6 +89,8 @@ def test_gptq_matches_reference(golden):
         gi = np.arange(k) // gsz
         w = (s.T[gi] * q - z.T[gi]).T  # [N, K]
         np.testing.assert_allclose(w, g[name + "_wdq"], rtol=0, atol=2e-7)
+        # packing the decoded integers again gives the reference's words bit for bit (any K, no group structure)
+        assert np.array_equal(ogptq.pack_values(ogptq.unpack_int4(qw, k), 4), qw), name
         bias = np.broadcast_to(g[name + "_bias"], x.shape[:-1] + (n,))
         y = ogptq.dequant_matmul(x, qw, bias, s, z, 0 if gs == -1 else gs)
         # reference pin: test_cuda_kernel.py:47  rtol = atol = 1e-5 against Linear(dequantised W)
@@ -258,6 +260,7 @@ def test_gptq_lowbit_matches_reference(golden):
         assert qw.shape[0] == ogptq.packed_rows(k, bit), name
         q = ogptq.unpack_bits(qw, k, bit)
         assert q.max() <= 2**bit - 1
+        assert np.array_equal(ogptq.pack_values(q, bit), qw), name
         gi = np.arange(k) // (k if gs == -1 else gs)
         w = (s.T[gi] * q.astype(np.float32) - z.T[gi]).T
         np.testing.assert_allclose(w, g[name + "_wdq"], rtol=0, atol=4e-7, err_msg=name)
